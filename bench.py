@@ -4,12 +4,17 @@
   python bench.py --gpus N --steps K --warmup W                 # B200 arm: MaskDiT-XL/2 ImageNet-256 train step
   python bench.py --impl reference --gpus N --steps K --warmup W  # reference arm: the CPU path of the same workload
   python bench.py --workload sampler                            # EDM sampler, 18 steps, CFG 1.5, batch 64
+  python bench.py ... --dump-outputs DIR                        # + what the last timed step computed, as DIR/*.npy
 
 A "step" = EDMLoss forward + hand-written backward + (N>1: one NCCL all-reduce of the flat fp32 gradient) +
 fused AdamW + EMA, on synthetic latents of BASELINE.json's shape with random-init XL/2 weights (the reference's
-zero-initialised tensors are randomised, SURVEY.md §3.3 — otherwise the net is the identity).
+zero-initialised tensors are randomised, SURVEY.md §3.3 — otherwise the net is the identity).  For the sampler
+workload a "step" is one whole 18-step sampler run.
 `value`  : samples/s, inputs resident in HBM.      `e2e.value`: same, inputs copied from pinned host memory
 every step and the loss read back to the host every step.
+
+Weights, inputs and the step's random draws are seeded, so the same arguments give the same inputs in every run and
+`--dump-outputs` of two builds can be compared array for array (up to floating-point summation order).
 """
 from __future__ import annotations
 
@@ -91,6 +96,34 @@ def randomise_zero_init(net, seed=1):
         for k, p in net.named_parameters():
             if p.requires_grad and float(p.abs().sum()) == 0.0:
                 p.copy_(torch.randn(p.shape, generator=g) * 0.02)
+
+
+DUMP_SAMPLE = 1 << 20   # elements drawn from each parameter-sized output: 4 MB per array in float32
+
+
+def sampled(named, n=DUMP_SAMPLE, seed=0):
+    """A fixed, seeded sample of n elements (with replacement, in index order) of the concatenation of the tensors in
+    `named` (registration order of the module, so the sample does not depend on how the library lays them out)."""
+    sizes = torch.tensor([t.numel() for _, t in named])
+    ends = sizes.cumsum(0)
+    idx = torch.randint(0, int(ends[-1]), (n,), generator=torch.Generator().manual_seed(seed)).sort().values
+    owner = torch.searchsorted(ends, idx, right=True)
+    parts = []
+    for j, (_, t) in enumerate(named):
+        local = idx[owner == j] - (ends[j] - sizes[j])
+        if len(local):
+            parts.append(t.detach().reshape(-1)[local.to(t.device)].float().cpu())
+    return torch.cat(parts).numpy()
+
+
+def write_outputs(d, arrays):
+    """DIR/<name>.npy for every array (float32 / float64 only)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 def make_batches(n, B, R, ncls, seed=0):
@@ -184,7 +217,7 @@ def have_unmodified_reference():
 
 
 def cpu_reference_train_unmodified(B, steps, warmup, R=32):
-    """The UNMODIFIED reference (`models/maskdit.py` + `train_utils/loss.py`, staged from /root/reference into the
+    """The UNMODIFIED reference (`models/maskdit.py` + `train_utils/loss.py`, staged from `MDT_REFERENCE_DIR` into the
     git-ignored baseline/_ref/ by `__graft_entry__.build()`), imported through the timm stand-in, fp32, PyTorch CPU backend,
     `torch.optim.AdamW(weight_decay=0)` in place of apex FusedAdam, the net wrapped to expose `.module` as the loss
     expects (loss.py:47) - BASELINE.md section 3.  Zero-initialised tensors randomised N(0, 0.02) like the GPU run."""
@@ -248,8 +281,8 @@ def cpu_baseline_record(steps, warmup, R=32, B=8, extras=False, prefer_unmodifie
     return sps, secs, {**extra, "value": sps, "unit": "samples/s", "cores": threads, "kind": "port", "same_config": False,
                        "sample": f"{steps} timed steps (+{warmup} warm-up) of batch {B} (SURVEY 8d), EDM loss fwd + bwd + "
                                  f"AdamW, torch CPU fp32, {threads} threads {how}; host has {os.cpu_count()} logical "
-                                 f"CPUs; {secs:.1f} s timed.  /root/reference is not on the GPU box: the oracle port "
-                                 "(pinned to the unmodified reference by tests/golden) is what runs"}
+                                 f"CPUs; {secs:.1f} s timed.  No unmodified reference staged in baseline/_ref: the "
+                                 "oracle port (pinned to the unmodified reference by tests/golden) is what runs"}
 
 
 def run_reference_arm(args, rank):
@@ -336,7 +369,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sub", action="store_true",
                     help="skip the sub-records (BASELINE configs 3-5: 128/GPU, 64x64x4 latents, sampler)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step of the headline workload computed "
+                         "as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -356,10 +394,10 @@ def main():
     R = 64 if args.workload == "train512" else 32
     net = build_xl2(R, dev)
     if args.workload == "sampler":
-        line = bench_sampler(args, net, env, PK)
+        line = bench_sampler(args, net, env, PK, dump=args.dump_outputs)
     else:
         line = bench_train(args, net, env, R, PK, args.batch_per_gpu or (256 if R == 32 else 128), args.steps,
-                           args.warmup, full=True)
+                           args.warmup, full=True, dump=args.dump_outputs)
         if args.workload == "train256" and not args.no_sub and args.batch_per_gpu is None:
             # BASELINE.json configs 3, 4, 5 next to the headline (config 2), same process, same box, same clocks
             # (a sub-record that fails - symmetrically on every rank, e.g. out of memory - must not cost the headline)
@@ -411,9 +449,11 @@ def main():
         dist.destroy_process_group()
 
 
-def bench_train(args, net, env, R, PK, B, steps, warmup, full):
+def bench_train(args, net, env, R, PK, B, steps, warmup, full, dump=None):
     """One training-step measurement.  full=True: the headline record (resident + e2e + per-launch GEMM timing +
-    clocks); full=False: a compact sub-record (resident inputs only)."""
+    clocks); full=False: a compact sub-record (resident inputs only).  dump: directory that receives what the last
+    timed (resident) step returned to its caller - the per-sample loss and the updated weights, EMA weights and
+    gradients (a seeded sample of each) - taken before any later step changes them."""
     import copy
 
     from maskdit_b200 import _lib
@@ -426,10 +466,11 @@ def bench_train(args, net, env, R, PK, B, steps, warmup, full):
     resident = [(x.to(dev), y.to(dev)) for x, y in pool]
     h2d = pool[0][0].numel() * 4 + pool[0][1].numel() * 4
     loss_host = torch.zeros(1).pin_memory()
+    last = {}
 
     def step_resident(i):
         x, y = resident[i % len(resident)]
-        return ts.step(x, y, 0.5, 0.1)
+        last["loss"] = ts.step(x, y, 0.5, 0.1)
 
     def step_e2e(i):
         xh, yh = pool[i % len(pool)]
@@ -446,6 +487,13 @@ def bench_train(args, net, env, R, PK, B, steps, warmup, full):
     ms = env.timed(step_resident, steps)
     launches = _lib.LAUNCHES - n0
     clk = clocks.stop() if (rank == 0 and full) else None
+    if dump and rank == 0:
+        trainable = [(k, p) for k, p in net.named_parameters() if p.requires_grad]
+        write_outputs(dump, {
+            "loss": last["loss"].float().cpu().numpy(),
+            "weights_sample": sampled(trainable),
+            "ema_weights_sample": sampled([(k, p) for k, p in ema.named_parameters() if p.requires_grad]),
+            "grads_sample": sampled([(k, p.grad) for k, p in trainable])})
     ms_step = ms / steps
     sps = B * world * steps / (ms / 1e3)
     flop = FLOP_PER_SAMPLE[256 if R == 32 else 512]
@@ -514,7 +562,8 @@ def bench_train(args, net, env, R, PK, B, steps, warmup, full):
     return line
 
 
-def bench_sampler(args, net, env, PK, iters=None, warm=None):
+def bench_sampler(args, net, env, PK, iters=None, warm=None, dump=None):
+    """`iters` sampler runs timed (default: --steps); dump: directory that receives the final latents of the last one."""
     from maskdit_b200 import _lib
     from maskdit_b200.sampler import edm_sampler
     dev, world, rank = env.dev, env.world, env.rank
@@ -534,12 +583,14 @@ def bench_sampler(args, net, env, PK, iters=None, warm=None):
     W = warm if warm is not None else max(1, args.warmup // 3)
     for i in range(W):
         run(i)
-    K = iters if iters is not None else max(1, args.steps // 5)
+    K = iters if iters is not None else args.steps
     clocks = ClockSampler(torch.cuda.current_device())
     if rank == 0:
         clocks.start()
     n0 = _lib.LAUNCHES
     ms = env.timed(run, K)
+    if dump and rank == 0:
+        write_outputs(dump, {"latents": out_h.numpy()})
     ips = B * world * K / (ms / 1e3)
     ach = ips / world * SAMPLER_FLOP_PER_IMAGE / 1e12
     return {"metric": "edm_sampler_imgs_per_sec", "value": ips, "unit": "img/s", "n_gpus": world, "steps": K,

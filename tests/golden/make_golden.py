@@ -1,6 +1,6 @@
-"""Generate golden vectors by executing the UNMODIFIED reference (/root/reference) on CPU fp32.
+"""Generate golden vectors by executing the UNMODIFIED reference (a checkout of the original MaskDiT) on CPU fp32.
 
-Run in the dev container only (the GPU box has no /root/reference):  python tests/golden/make_golden.py
+    MDT_REFERENCE_DIR=<checkout of Anima-Lab/MaskDiT> python tests/golden/make_golden.py
 Writes tests/golden/*.npz (small).  Weights are NOT stored: both the reference module and the oracle are loaded
 from oracle.maskdit_oracle.make_state_dict(cfg, seed) which is deterministic on CPU.
 
@@ -20,7 +20,9 @@ from oracle import maskdit_oracle as O  # noqa: E402
 from oracle import timm_standin  # noqa: E402
 
 timm_standin.install()
-sys.path.insert(0, "/root/reference")
+if not os.path.isdir(os.environ.get("MDT_REFERENCE_DIR", "")):
+    sys.exit("set MDT_REFERENCE_DIR to a checkout of the original MaskDiT (models/maskdit.py, train_utils/loss.py, ...)")
+sys.path.insert(0, os.environ["MDT_REFERENCE_DIR"])
 import models.maskdit as rm  # noqa: E402
 import sample as rs  # noqa: E402
 import train_utils.loss as rl  # noqa: E402
