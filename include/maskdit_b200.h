@@ -308,10 +308,11 @@ int mdt_nccl_comm_destroy(void* comm);
 int mdt_allreduce_grads(void* comm, void* grad, long long n, int bf16, void* stream);
 
 /* ============================================================================================================
- * Sampler tail: SD-VAE decode (sample.py:275 `vae.decode(z)`; autoencoder.py:306-453).  Activations are pixel-major
- * fp32 row matrices [B*H*W, C]; every convolution is mdt_gemm_bf16 on an im2col operand built by mdt_vae_im2col with
- * the GroupNorm(32) affine, the swish and the nearest-2x upsample of its source fused in.  The host sequencing is
- * maskdit_b200/vae.py (same state-dict keys as FrozenAutoencoderKL: `decoder.*`, `post_quant_conv.*`).
+ * SD-VAE: decode, the sampler tail (sample.py:275 `vae.decode(z)`; autoencoder.py:306-453), and encode_moments, the
+ * latent extraction in front of training (extract_latent.py:77; autoencoder.py:212-303,431-434).  Activations are
+ * pixel-major fp32 row matrices [B*H*W, C]; every convolution is mdt_gemm_bf16 on an im2col operand built by
+ * mdt_vae_im2col (GroupNorm(32) affine, swish and nearest-2x upsample of its source fused in) or mdt_vae_im2col_down.
+ * The host sequencing is maskdit_b200/vae.py (same state-dict keys as FrozenAutoencoderKL).
  * ============================================================================================================ */
 /* out [B*P, C] f32 = post_quant_conv(z / scale_factor), z [B,C,h,w] NCHW (autoencoder.py:449-451); C <= 8           */
 int mdt_vae_post_quant(const float* z, const float* W, const float* bias, float scale_factor, float* out, int B,
@@ -324,8 +325,21 @@ int mdt_vae_gn_stats(const float* x, double* sums, float* scratch, int B, int P,
  * norm_out inputs (autoencoder.py:49-53,117-137,404-406); columns >= ks*ks*C are zero.                              */
 int mdt_vae_im2col(const float* src, const double* sums, const float* gamma, const float* beta, int silu, int ks,
                    int up, void* A_bf16, int B, int H, int W, int C, int Kp, void* stream);
+/* A [B*(H/2)*(W/2), Kp] bf16, A[(b,y,x),(ky,kx,c)] = src[b,2y+ky,2x+kx,c], 0 where 2y+ky >= H or 2x+kx >= W: the
+ * F.pad(x,(0,1,0,1)) + 3x3 stride-2 convolution of Downsample (autoencoder.py:56-75).  src [B,H,W,C] f32 (H, W: source
+ * dims, even); columns >= 9*C are zero.                                                                              */
+int mdt_vae_im2col_down(const float* src, void* A_bf16, int B, int H, int W, int C, int Kp, void* stream);
+/* x [B,3,H,W] f32 NCHW -> out [B*H*W, 4] f32 pixel-major rows, channel 3 = 0 (the encoder's conv_in input);
+ * flip != 0 mirrors x along W (`img.flip(dims=[-1])`, extract_latent.py:85)                                          */
+int mdt_vae_image_to_rows(const float* x, float* out, int B, int H, int W, int flip, void* stream);
+/* moments [B,C,P] f32 NCHW = quant_conv(rows) (1x1, autoencoder.py:431-434), rows [B*P, ldx] f32 (first C columns); C <= 8 */
+int mdt_vae_quant_out(const float* rows, int ldx, const float* W, const float* bias, float* moments, int B, int C,
+                      int P, void* stream);
 /* P [rows, cols] bf16 = softmax(scale * S) along columns (AttnBlock, autoencoder.py:185-187)                        */
 int mdt_vae_softmax_rows(const float* S, float scale, void* P_bf16, int rows, int cols, void* stream);
+/* the same with row stride ld >= cols for S and P; P[:, cols:ld] = 0 (T = h*w not a multiple of 8: the GEMMs need
+ * 16-byte row strides)                                                                                                */
+int mdt_vae_softmax_rows_ld(const float* S, float scale, void* P_bf16, int rows, int cols, int ld, void* stream);
 /* x [B,P,ldx] f32 (first C columns) -> out [B,C,P] f32: the NCHW image `decode` returns                             */
 int mdt_vae_rows_to_nchw(const float* x, float* out, int B, int P, int C, int ldx, void* stream);
 

@@ -105,6 +105,10 @@ _SIGS = {
     "mdt_vae_gn_stats": [_P, _P, _P, _I, _I, _I, _P],
     "mdt_vae_im2col": [_P, _P, _P, _P, _I, _I, _I, _P, _I, _I, _I, _I, _I, _P],
     "mdt_vae_softmax_rows": [_P, _F, _P, _I, _I, _P],
+    "mdt_vae_softmax_rows_ld": [_P, _F, _P, _I, _I, _I, _P],
+    "mdt_vae_im2col_down": [_P, _P, _I, _I, _I, _I, _I, _P],
+    "mdt_vae_image_to_rows": [_P, _P, _I, _I, _I, _I, _P],
+    "mdt_vae_quant_out": [_P, _I, _P, _P, _P, _I, _I, _I, _P],
     "mdt_vae_rows_to_nchw": [_P, _P, _I, _I, _I, _I, _P],
     "mdt_adamw_ema_g16": [_P, _P, _P, _P, _P, _P, _LL, _F, _F, _F, _F, _F, _I, _F, _F, _I, _P],
     "mdt_set_sm_budget": [_I],

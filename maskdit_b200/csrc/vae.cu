@@ -1,6 +1,8 @@
 // Sampler tail: the SD-VAE DECODE path the reference runs on every batch of sampled latents (sample.py:275
 // `images = vae.decode(z)`; autoencoder.py:306-453: post_quant_conv, conv_in, ResnetBlocks with GroupNorm(32)+swish,
-// one single-head AttnBlock, nearest-2x Upsample + conv, norm_out + conv_out).
+// one single-head AttnBlock, nearest-2x Upsample + conv, norm_out + conv_out), and the ENCODE path in front of training
+// (extract_latent.py:77 `encode_moments`; autoencoder.py:212-303,431-434: conv_in on the 3-channel image, ResnetBlocks,
+// stride-2 Downsample convolutions with (0,1,0,1) padding, the AttnBlock, norm_out + conv_out, quant_conv).
 //
 // Layout: activations are pixel-major ("NHWC") fp32 row matrices [B*H*W, C], so every convolution is a GEMM on the
 // tcgen05 kernel of gemm_tcgen05.cu: a 3x3 convolution reads an im2col operand A[(b,y,x), (ky,kx,c)] (bf16) that ONE
@@ -77,15 +79,20 @@ __global__ void vae_gn_finish_kernel(const float* __restrict__ partial, double* 
 //   f = identity | GroupNorm affine (sums / gamma / beta given) | GroupNorm affine then swish (silu != 0)
 //   ks = 3 (pad 1) or 1 (pad 0);  up = 1 or 2 (nearest upsample of the source, Upsample.forward autoencoder.py:49-53)
 //   src [B, H/up, W/up, C] f32  ->  A [B*H*W, Kp] bf16,  Kp >= ks*ks*C (extra columns zero)
+// Downsample mode (down != 0; ks = 3, up = 1, f = identity): the output grid is H/2 x W/2 and
+//   A[(b, y, x), (ky, kx, c)] = src[b, 2y+ky, 2x+kx, c], zero where 2y+ky >= H or 2x+kx >= W
+//   = F.pad(x, (0,1,0,1)) then the 3x3 stride-2 convolution of Downsample.forward (autoencoder.py:56-75).
 // Thread = 4 channels; blockDim = (C/4, 256/(C/4)) (C = 4: 1 x 256); each y-lane walks output pixels.
 __global__ void __launch_bounds__(256)
 vae_im2col_kernel(const float* __restrict__ src, const double* __restrict__ sums, const float* __restrict__ gamma,
-                  const float* __restrict__ beta, int silu_on, int ks, int up, __nv_bfloat16* __restrict__ A, int B,
-                  int H, int W, int C, int Kp, float eps) {
+                  const float* __restrict__ beta, int silu_on, int ks, int up, int down, __nv_bfloat16* __restrict__ A,
+                  int B, int H, int W, int C, int Kp, float eps) {
   const int tx = threadIdx.x, c = 4 * tx;
-  const int Hs = H / up, Ws = W / up;
-  const long long npix = static_cast<long long>(B) * H * W;
-  const int pad = ks / 2, taps = ks * ks;
+  const int Hs = H / up, Ws = W / up;                  // source dims (H, W: the source dims in downsample mode)
+  const int Ho = down ? H / 2 : H, Wo = down ? W / 2 : W;
+  const int stride = down ? 2 : 1;
+  const long long npix = static_cast<long long>(B) * Ho * Wo;
+  const int pad = down ? 0 : ks / 2, taps = ks * ks;
   float4 ga = make_float4(1.f, 1.f, 1.f, 1.f), be = make_float4(0.f, 0.f, 0.f, 0.f);
   if (sums) {
     ga = *reinterpret_cast<const float4*>(gamma + c);
@@ -95,9 +102,9 @@ vae_im2col_kernel(const float* __restrict__ src, const double* __restrict__ sums
   const double cnt = static_cast<double>(Hs) * Ws * cg;
   for (long long pix = blockIdx.x * static_cast<long long>(blockDim.y) + threadIdx.y; pix < npix;
        pix += static_cast<long long>(gridDim.x) * blockDim.y) {
-    const int b = static_cast<int>(pix / (static_cast<long long>(H) * W));
-    const int yx = static_cast<int>(pix - static_cast<long long>(b) * H * W);
-    const int y = yx / W, x = yx - y * W;
+    const int b = static_cast<int>(pix / (static_cast<long long>(Ho) * Wo));
+    const int yx = static_cast<int>(pix - static_cast<long long>(b) * Ho * Wo);
+    const int y = yx / Wo, x = yx - y * Wo;
     float mean = 0.f, rstd = 1.f;
     if (sums) {
       const int g = c / cg;
@@ -109,7 +116,7 @@ vae_im2col_kernel(const float* __restrict__ src, const double* __restrict__ sums
     __nv_bfloat16* arow = A + pix * Kp;
     for (int t = 0; t < taps; ++t) {
       const int ky = t / ks, kx = t - ky * ks;
-      const int sy = y + ky - pad, sx = x + kx - pad;
+      const int sy = stride * y + ky - pad, sx = stride * x + kx - pad;
       uint2 o = make_uint2(0u, 0u);
       if (sy >= 0 && sy < H && sx >= 0 && sx < W) {
         const float4 v = *reinterpret_cast<const float4*>(
@@ -129,20 +136,53 @@ vae_im2col_kernel(const float* __restrict__ src, const double* __restrict__ sums
   }
 }
 
-// P[r, :] = softmax(scale * S[r, :]) as bf16; one warp per row (AttnBlock, autoencoder.py:186-187)
+// x [B,3,H,W] f32 NCHW (the normalised image batch) -> out [B*H*W, 4] f32 pixel-major rows, channel 3 = 0, so that
+// conv_in (autoencoder.py:230-234) is the im2col GEMM with C = 4.  flip != 0 reads x mirrored along W (the xflip pass
+// of extract_latent.py:85, `img.flip(dims=[-1])`).
+__global__ void vae_image_to_rows_kernel(const float* __restrict__ x, float* __restrict__ out, int B, int H, int W,
+                                         int flip) {
+  const long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;  // (b, y, x)
+  const long long P = static_cast<long long>(H) * W;
+  if (i >= B * P) return;
+  const int b = static_cast<int>(i / P), yx = static_cast<int>(i - b * P);
+  const int y = yx / W, xx = yx - y * W;
+  const long long s = static_cast<long long>(b) * 3 * P + static_cast<long long>(y) * W + (flip ? W - 1 - xx : xx);
+  *reinterpret_cast<float4*>(out + 4 * i) = make_float4(x[s], x[s + P], x[s + 2 * P], 0.f);
+}
+
+// rows [B*P, ldx] f32 (encoder conv_out, first C columns valid) -> moments [B,C,P] f32 NCHW = quant_conv (1x1, C -> C)
+// (FrozenAutoencoderKL.encode_moments, autoencoder.py:431-434); C <= 8
+__global__ void vae_quant_out_kernel(const float* __restrict__ rows, int ldx, const float* __restrict__ Wq,
+                                     const float* __restrict__ bias, float* __restrict__ moments, int B, int C, int P) {
+  const long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;  // (b, pixel)
+  if (i >= static_cast<long long>(B) * P) return;
+  const int b = static_cast<int>(i / P), p = static_cast<int>(i % P);
+  float v[8];
+  for (int c = 0; c < C; ++c) v[c] = rows[i * ldx + c];
+  for (int o = 0; o < C; ++o) {
+    float acc = bias[o];
+    for (int c = 0; c < C; ++c) acc = fmaf(Wq[o * C + c], v[c], acc);
+    moments[(static_cast<long long>(b) * C + o) * P + p] = acc;
+  }
+}
+
+// P[r, :cols] = softmax(scale * S[r, :cols]) as bf16, P[r, cols:ld] = 0; S and P have row stride ld >= cols; one
+// warp per row (AttnBlock, autoencoder.py:186-187)
 __global__ void __launch_bounds__(256)
-vae_softmax_rows_kernel(const float* __restrict__ S, float scale, __nv_bfloat16* __restrict__ P, int rows, int cols) {
+vae_softmax_rows_kernel(const float* __restrict__ S, float scale, __nv_bfloat16* __restrict__ P, int rows, int cols,
+                        int ld) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (row >= rows) return;
-  const float* s = S + static_cast<long long>(row) * cols;
+  const float* s = S + static_cast<long long>(row) * ld;
   float mx = -INFINITY;
   for (int j = lane; j < cols; j += 32) mx = fmaxf(mx, s[j]);
   mx = warp_max(mx);
   float sum = 0.f;
   for (int j = lane; j < cols; j += 32) sum += __expf(scale * (s[j] - mx));
   const float inv = 1.f / warp_sum(sum);
-  __nv_bfloat16* p = P + static_cast<long long>(row) * cols;
+  __nv_bfloat16* p = P + static_cast<long long>(row) * ld;
   for (int j = lane; j < cols; j += 32) p[j] = __float2bfloat16_rn(__expf(scale * (s[j] - mx)) * inv);
+  for (int j = cols + lane; j < ld; j += 32) p[j] = __float2bfloat16_rn(0.f);
 }
 
 // x [B, P, ldx] f32 (first C columns valid) -> out [B, C, P] f32 (the [B,3,H,W] image the reference's decode returns)
@@ -191,14 +231,51 @@ int mdt_vae_im2col(const float* src, const double* sums, const float* gamma, con
   long long blocks = (npix + ty - 1) / ty;
   if (blocks > 148 * 16) blocks = 148 * 16;
   vae_im2col_kernel<<<static_cast<int>(blocks), dim3(tx, ty), 0, VS(stream)>>>(
-      src, sums, gamma, beta, silu, ks, up, static_cast<__nv_bfloat16*>(A_bf16), B, H, W, C, Kp, 1e-6f);
+      src, sums, gamma, beta, silu, ks, up, 0, static_cast<__nv_bfloat16*>(A_bf16), B, H, W, C, Kp, 1e-6f);
+  return vae_status();
+}
+
+int mdt_vae_im2col_down(const float* src, void* A_bf16, int B, int H, int W, int C, int Kp, void* stream) {
+  if (!src || !A_bf16 || B <= 0 || H <= 0 || W <= 0 || H % 2 || W % 2 || C % 4 || C > 1024 || Kp < 9 * C || Kp % 8)
+    return MDT_ERR_ARG;
+  if ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(A_bf16)) & 15) return MDT_ERR_ARG;
+  const int tx = C / 4, ty = tx >= 256 ? 1 : 256 / tx;
+  const long long npix = static_cast<long long>(B) * (H / 2) * (W / 2);
+  long long blocks = (npix + ty - 1) / ty;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  vae_im2col_kernel<<<static_cast<int>(blocks), dim3(tx, ty), 0, VS(stream)>>>(
+      src, nullptr, nullptr, nullptr, 0, 3, 1, 1, static_cast<__nv_bfloat16*>(A_bf16), B, H, W, C, Kp, 1e-6f);
+  return vae_status();
+}
+
+int mdt_vae_image_to_rows(const float* x, float* out, int B, int H, int W, int flip, void* stream) {
+  if (!x || !out || B <= 0 || H <= 0 || W <= 0) return MDT_ERR_ARG;
+  if (reinterpret_cast<uintptr_t>(out) & 15) return MDT_ERR_ARG;
+  const long long n = static_cast<long long>(B) * H * W;
+  vae_image_to_rows_kernel<<<static_cast<int>((n + 255) / 256), 256, 0, VS(stream)>>>(x, out, B, H, W, flip);
+  return vae_status();
+}
+
+int mdt_vae_quant_out(const float* rows, int ldx, const float* W, const float* bias, float* moments, int B, int C,
+                      int P, void* stream) {
+  if (!rows || !W || !bias || !moments || B <= 0 || C <= 0 || C > 8 || P <= 0 || ldx < C) return MDT_ERR_ARG;
+  const long long n = static_cast<long long>(B) * P;
+  vae_quant_out_kernel<<<static_cast<int>((n + 255) / 256), 256, 0, VS(stream)>>>(rows, ldx, W, bias, moments, B, C,
+                                                                                 P);
   return vae_status();
 }
 
 int mdt_vae_softmax_rows(const float* S, float scale, void* P_bf16, int rows, int cols, void* stream) {
   if (!S || !P_bf16 || rows <= 0 || cols <= 0) return MDT_ERR_ARG;
   vae_softmax_rows_kernel<<<(rows + 7) / 8, 256, 0, VS(stream)>>>(S, scale, static_cast<__nv_bfloat16*>(P_bf16), rows,
-                                                                  cols);
+                                                                  cols, cols);
+  return vae_status();
+}
+
+int mdt_vae_softmax_rows_ld(const float* S, float scale, void* P_bf16, int rows, int cols, int ld, void* stream) {
+  if (!S || !P_bf16 || rows <= 0 || cols <= 0 || ld < cols) return MDT_ERR_ARG;
+  vae_softmax_rows_kernel<<<(rows + 7) / 8, 256, 0, VS(stream)>>>(S, scale, static_cast<__nv_bfloat16*>(P_bf16), rows,
+                                                                  cols, ld);
   return vae_status();
 }
 

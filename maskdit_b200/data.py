@@ -9,7 +9,8 @@ into the float one-hot the label embedder consumes.
 The `lmdb` Python module is not part of this image, so `MdbReader` below is a read-only walker of LMDB's on-disk
 B+tree (`data.mdb`: two meta pages, branch / leaf / overflow pages) written from the published file format; when
 `lmdb` IS importable it is used instead.  PARITY UNPINNED against liblmdb itself (no liblmdb here to produce a
-fixture): `tests/test_data.py` round-trips files produced by `write_mdb` (the same format, bulk-loaded).
+fixture): `tests/test_data.py` round-trips files produced by `write_mdb` / `MdbWriter` (the same format; `MdbWriter`
+streams overflow values to disk, so a 1.28 M-image ImageNet extraction never holds its ~42 GB of moments in memory).
 
 Nothing here runs on the GPU: batches are assembled in pinned host memory and copied by the caller; the arithmetic
 that follows (moments -> latent, label dropout, noise injection) is `ops.step_front` (csrc/loss_optim.cu).
@@ -106,21 +107,56 @@ class MdbReader:
             return None
 
 
-def write_mdb(path, items, psize=4096):
-    """Bulk-load `items` (dict bytes -> bytes) into a fresh single-database LMDB file `<path>/data.mdb` (tests and
-    synthetic datasets; the reference writes these with liblmdb, extract_latent.py:60-106)."""
-    os.makedirs(path, exist_ok=True)
-    keys = sorted(items)
-    pages = {}          # pgno -> bytes
-    next_pg = [2]
-    n_leaf = n_branch = n_over = 0
+def _node(key, size, flags, payload):
+    """Leaf node: (size lo, size hi, flags, key size), key, then the value (or the first overflow pgno, F_BIGDATA)."""
+    return struct.pack("<HHHH", size & 0xFFFF, size >> 16, flags, len(key)) + key + payload
 
-    def alloc(n=1):
-        p = next_pg[0]
-        next_pg[0] += n
-        return p
 
-    def build_page(pgno, flags, nodes):
+def _branch_node(key, pgno):
+    return struct.pack("<HHHH", pgno & 0xFFFF, (pgno >> 16) & 0xFFFF, (pgno >> 32) & 0xFFFF, len(key)) + key
+
+
+class MdbWriter:
+    """Stream a fresh single-database LMDB file `<path>/data.mdb` (the layout extract_latent.py:60-106 writes with
+    liblmdb).  `put(key, value)` appends values too large for a leaf node (every VAE moment) to the file at once as
+    overflow pages; only `(key, pgno, length)` records and small inline values stay in memory.  `close()` builds the
+    sorted leaf and branch pages after them and then writes the two meta pages at offsets 0 and psize.  Keys may come
+    in any order; a key can be put once."""
+
+    def __init__(self, path, psize=4096):
+        os.makedirs(path, exist_ok=True)
+        self.psize = psize
+        self._f = open(os.path.join(path, "data.mdb"), "wb")
+        self._f.write(bytes(2 * psize))          # meta pages 0 and 1, written by close()
+        self._next = 2                           # next free page number
+        self._nodes = {}                         # key -> leaf node bytes
+        self._n_over = 0
+
+    def _write_pages(self, buf):
+        assert len(buf) % self.psize == 0
+        pg = self._next
+        self._f.write(buf)
+        self._next += len(buf) // self.psize
+        return pg
+
+    def put(self, key, value):
+        key, value = bytes(key), bytes(value)
+        if key in self._nodes:
+            raise KeyError(f"MdbWriter: key {key!r} was already put")
+        psize = self.psize
+        if 8 + len(key) + len(value) > psize // 2 - PAGEHDR:        # value goes to overflow pages
+            npg = (PAGEHDR + len(value) + psize - 1) // psize
+            buf = bytearray(npg * psize)
+            struct.pack_into("<QHHI", buf, 0, self._next, 0, P_OVERFLOW, npg)
+            buf[PAGEHDR:PAGEHDR + len(value)] = value
+            ov = self._write_pages(buf)
+            self._n_over += npg
+            self._nodes[key] = _node(key, len(value), F_BIGDATA, struct.pack("<Q", ov))
+        else:
+            self._nodes[key] = _node(key, len(value), 0, value)
+
+    def _page(self, flags, nodes):
+        psize = self.psize
         buf = bytearray(psize)
         upper = psize
         ptrs = []
@@ -130,81 +166,94 @@ def write_mdb(path, items, psize=4096):
             ptrs.append(upper)
         lower = PAGEHDR + 2 * len(ptrs)
         assert lower <= upper
-        struct.pack_into("<QHHHH", buf, 0, pgno, 0, flags, lower, upper)
+        struct.pack_into("<QHHHH", buf, 0, self._next, 0, flags, lower, upper)
         struct.pack_into(f"<{len(ptrs)}H", buf, PAGEHDR, *ptrs)
-        pages[pgno] = bytes(buf)
+        return self._write_pages(buf)
 
-    def fits(nodes, nd):
-        used = sum(len(x) + (len(x) & 1) for x in nodes) + len(nd) + (len(nd) & 1)
-        return PAGEHDR + 2 * (len(nodes) + 1) + used <= psize
+    def _fits(self, nodes, used, nd):
+        return PAGEHDR + 2 * (len(nodes) + 1) + used + len(nd) + (len(nd) & 1) <= self.psize
 
-    nodemax = psize // 2 - PAGEHDR
-    level = []          # (first key, pgno)
-    cur, first = [], None
-    for k in keys:
-        v = items[k]
-        if 8 + len(k) + len(v) > nodemax:                          # value goes to overflow pages
-            npg = (PAGEHDR + len(v) + psize - 1) // psize
-            ov = alloc(npg)
-            buf = bytearray(npg * psize)
-            struct.pack_into("<QHHI", buf, 0, ov, 0, P_OVERFLOW, npg)
-            buf[PAGEHDR:PAGEHDR + len(v)] = v
-            for j in range(npg):
-                pages[ov + j] = bytes(buf[j * psize:(j + 1) * psize])
-            n_over += npg
-            nd = struct.pack("<HHHH", len(v) & 0xFFFF, len(v) >> 16, F_BIGDATA, len(k)) + k + struct.pack("<Q", ov)
-        else:
-            nd = struct.pack("<HHHH", len(v) & 0xFFFF, len(v) >> 16, 0, len(k)) + k + v
-        if cur and not fits(cur, nd):
-            pg = alloc()
-            build_page(pg, P_LEAF, cur)
-            level.append((first, pg))
-            n_leaf += 1
-            cur, first = [], None
-        if first is None:
-            first = k
-        cur.append(nd)
-    if cur:
-        pg = alloc()
-        build_page(pg, P_LEAF, cur)
-        level.append((first, pg))
-        n_leaf += 1
-    depth = 1 if level else 0
-    while len(level) > 1:
-        nxt, cur, first = [], [], None
-        for k, pg in level:
-            kk = b"" if not cur else k
-            nd = struct.pack("<HHHH", pg & 0xFFFF, (pg >> 16) & 0xFFFF, (pg >> 32) & 0xFFFF, len(kk)) + kk
-            if cur and not fits(cur, nd):
-                bp = alloc()
-                build_page(bp, P_BRANCH, cur)
-                nxt.append((first, bp))
-                n_branch += 1
-                cur, first = [], None
-                nd = struct.pack("<HHHH", pg & 0xFFFF, (pg >> 16) & 0xFFFF, (pg >> 32) & 0xFFFF, 0)
+    def close(self):
+        if self._f is None:
+            return
+        psize = self.psize
+        keys = sorted(self._nodes)
+        n_leaf = n_branch = 0
+        level = []          # (first key, pgno)
+        cur, used, first = [], 0, None
+        for k in keys:
+            nd = self._nodes.pop(k)
+            if cur and not self._fits(cur, used, nd):
+                level.append((first, self._page(P_LEAF, cur)))
+                n_leaf += 1
+                cur, used, first = [], 0, None
             if first is None:
                 first = k
             cur.append(nd)
-        bp = alloc()
-        build_page(bp, P_BRANCH, cur)
-        nxt.append((first, bp))
-        n_branch += 1
-        level = nxt
-        depth += 1
-    root = level[0][1] if level else P_INVALID
-    last_pg = next_pg[0] - 1
-    for m in (0, 1):
-        buf = bytearray(psize)
-        struct.pack_into("<QHHI", buf, 0, m, 0, P_META, 0)
-        b = PAGEHDR
-        struct.pack_into("<IIQQ", buf, b, MDB_MAGIC, 1, 0, max(1 << 20, (last_pg + 1) * psize))
-        struct.pack_into("<IHHQQQQQ", buf, b + 24, psize, 0, 0, 0, 0, 0, 0, P_INVALID)        # free DB (empty)
-        struct.pack_into("<IHHQQQQQ", buf, b + 72, 0, 0, depth, n_branch, n_leaf, n_over, len(keys), root)
-        struct.pack_into("<QQ", buf, b + 120, last_pg, 1 if m == 1 else 0)
-        pages[m] = bytes(buf)
-    with open(os.path.join(path, "data.mdb"), "wb") as f:
-        for pg in range(next_pg[0]):
-            f.write(pages[pg])
+            used += len(nd) + (len(nd) & 1)
+        if cur:
+            level.append((first, self._page(P_LEAF, cur)))
+            n_leaf += 1
+        depth = 1 if level else 0
+        while len(level) > 1:
+            nxt, cur, used, first = [], [], 0, None
+            for k, pg in level:
+                nd = _branch_node(b"" if not cur else k, pg)     # node 0 of a branch page has an empty key
+                if cur and not self._fits(cur, used, nd):
+                    nxt.append((first, self._page(P_BRANCH, cur)))
+                    n_branch += 1
+                    cur, used, first = [], 0, None
+                    nd = _branch_node(b"", pg)
+                if first is None:
+                    first = k
+                cur.append(nd)
+                used += len(nd) + (len(nd) & 1)
+            nxt.append((first, self._page(P_BRANCH, cur)))
+            n_branch += 1
+            level = nxt
+            depth += 1
+        root = level[0][1] if level else P_INVALID
+        last_pg = self._next - 1
+        for m in (0, 1):
+            buf = bytearray(psize)
+            struct.pack_into("<QHHI", buf, 0, m, 0, P_META, 0)
+            b = PAGEHDR
+            struct.pack_into("<IIQQ", buf, b, MDB_MAGIC, 1, 0, max(1 << 20, (last_pg + 1) * psize))
+            struct.pack_into("<IHHQQQQQ", buf, b + 24, psize, 0, 0, 0, 0, 0, 0, P_INVALID)        # free DB (empty)
+            struct.pack_into("<IHHQQQQQ", buf, b + 72, 0, 0, depth, n_branch, n_leaf, self._n_over, len(keys), root)
+            struct.pack_into("<QQ", buf, b + 120, last_pg, 1 if m == 1 else 0)
+            self._f.seek(m * psize)
+            self._f.write(buf)
+        self._f.close()
+        self._f = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+def write_mdb(path, items, psize=4096):
+    """Bulk-load `items` (dict bytes -> bytes) into a fresh single-database LMDB file `<path>/data.mdb` (tests and
+    synthetic datasets) through `MdbWriter`."""
+    with MdbWriter(path, psize) as w:
+        for k in sorted(items):
+            w.put(k, items[k])
+
+
+def center_crop_arr(pil_image, image_size):
+    """The reference's image preprocessing (train_utils/datasets.py:19-37, ADM's center crop): halve with BOX filtering
+    while the short side is at least twice `image_size`, resize with BICUBIC so the short side is `image_size`, then crop
+    the centre square.  Returns a PIL image of `image_size` x `image_size`."""
+    from PIL import Image
+    img = pil_image
+    while min(img.size) >= 2 * image_size:
+        img = img.resize((img.width // 2, img.height // 2), resample=Image.BOX)
+    s = image_size / min(img.size)
+    img = img.resize((round(img.width * s), round(img.height * s)), resample=Image.BICUBIC)
+    top, left = (img.height - image_size) // 2, (img.width - image_size) // 2
+    return Image.fromarray(np.asarray(img)[top:top + image_size, left:left + image_size])
 
 
 def write_latent_lmdb(root, moments, labels, split="train"):
