@@ -318,7 +318,9 @@ int mdt_allreduce_grads(void* comm, void* grad, long long n, int bf16, void* str
 int mdt_vae_post_quant(const float* z, const float* W, const float* bias, float scale_factor, float* out, int B,
                        int C, int P, void* stream);
 /* GroupNorm(32) statistics (Normalize, autoencoder.py:34-35) of x [B,P,C] f32: sums [B,32,2] f64 = (sum, sum of squares),
- * deterministic (fixed-order two-pass reduction); scratch: B * ceil(P/256) * 64 floats                              */
+ * deterministic (fixed-order two-pass reduction, accumulated about one sample of each group so that a large mean does
+ * not cancel the variance); C = 128, 256 or 512 (the VAE's widths; anything else is MDT_ERR_ARG);
+ * scratch: B * ceil(P/256) * 64 floats                                                                               */
 int mdt_vae_gn_stats(const float* x, double* sums, float* scratch, int B, int P, int C, void* stream);
 /* A [B*H*W, Kp] bf16, A[(b,y,x),(ky,kx,c)] = f(src[b,(y+ky-pad)/up,(x+kx-pad)/up,c]) (0 outside); ks = 1 | 3; up = 1 | 2;
  * f = identity (sums NULL) | GroupNorm affine | GroupNorm affine + swish (silu != 0): ResnetBlock / Upsample /

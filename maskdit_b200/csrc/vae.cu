@@ -38,24 +38,31 @@ __global__ void vae_post_quant_kernel(const float* __restrict__ z, const float* 
 
 // GroupNorm(32) statistics of x [B, P, C] f32, DETERMINISTIC (no atomics: with bf16 GEMM operands downstream, 1e-7
 // order noise in a mean flips bf16 roundings and shows up as 4e-3 run-to-run differences in the decoded image, measured):
-//   pass 1: block (b, chunk of kGnPix pixels) -> partial[b][chunk][g] = (sum, sum of squares) fp32, fixed-order tree
-//   pass 2: sums[b][g] = fixed-order fp64 sum of the partials.
-// Thread = 4 channels of one pixel lane; block = C/4 x (256 / (C/4)) threads: always 8 threads per group.
+//   pass 1: block (b, chunk of kGnPix pixels) -> partial[b][chunk][g] = (sum, sum of squares) of x - k_g fp32,
+//           fixed-order tree, with the shift k_g = x[b, pixel 0, first channel of group g] (one sample of the group)
+//   pass 2: sums[b][g] = fixed-order fp64 sum of the partials, shifted back to the (sum, sum of squares) of x.
+// Without the shift the fp32 sum of squares of a group whose mean is large against its spread cancels in q/n - m^2
+// (measured on a B200: rstd off by up to 7.6e-3 relative at mean / std = 100 to 200; 2e-6 with the shift).  Every
+// block reads the same k_g, so the result stays deterministic.
+// Thread = 4 channels of one pixel lane; block = C/4 x (256 / (C/4)) threads: 8 threads per group, so C is 128, 256 or
+// 512.
 constexpr int kGnPix = 256;
 __global__ void __launch_bounds__(256)
 vae_gn_partial_kernel(const float* __restrict__ x, float* __restrict__ partial, int P, int C) {
   __shared__ float s_part[256][2];
   const int tx = threadIdx.x, ty = threadIdx.y, b = blockIdx.y;
   const int p0 = blockIdx.x * kGnPix;
+  const int tpg = (C / 32) / 4;                       // threads per group along x (1, 2 or 4)
+  const int g = tx / tpg, member = ty * tpg + (tx - g * tpg);
+  const float kg = x[static_cast<long long>(b) * P * C + g * (C / 32)];
   float s = 0.f, ss = 0.f;
   for (int p = p0 + ty; p < min(P, p0 + kGnPix); p += blockDim.y) {
-    const float4 v = *reinterpret_cast<const float4*>(x + (static_cast<long long>(b) * P + p) * C + 4 * tx);
+    float4 v = *reinterpret_cast<const float4*>(x + (static_cast<long long>(b) * P + p) * C + 4 * tx);
+    v.x -= kg, v.y -= kg, v.z -= kg, v.w -= kg;
     s += (v.x + v.y) + (v.z + v.w);
     ss += (v.x * v.x + v.y * v.y) + (v.z * v.z + v.w * v.w);
   }
   // slot = (group, member): the 8 threads of a group occupy 8 consecutive slots
-  const int tpg = (C / 32) / 4;                       // threads per group along x (1, 2 or 4)
-  const int g = tx / tpg, member = ty * tpg + (tx - g * tpg);
   s_part[g * 8 + member][0] = s;
   s_part[g * 8 + member][1] = ss;
   __syncthreads();
@@ -68,11 +75,30 @@ vae_gn_partial_kernel(const float* __restrict__ x, float* __restrict__ partial, 
     partial[((static_cast<long long>(b) * gridDim.x + blockIdx.x) * 32 + gg) * 2 + w] = acc;
   }
 }
-__global__ void vae_gn_finish_kernel(const float* __restrict__ partial, double* __restrict__ sums, int nchunk) {
-  const int b = blockIdx.x, t = threadIdx.x;  // 64 threads: (group, which)
+// Block b = kGnLanes x 64 threads: lane l sums chunks l, l + kGnLanes, ... of value (group, which); the lanes are then
+// added in lane order (fixed, so deterministic).  Several lanes because the grid is only B blocks: latency-bound.
+constexpr int kGnLanes = 8;
+__global__ void __launch_bounds__(kGnLanes * 64)
+vae_gn_finish_kernel(const float* __restrict__ x, const float* __restrict__ partial, double* __restrict__ sums,
+                     int nchunk, int P, int C) {
+  __shared__ double s_acc[kGnLanes][64];
+  const int b = blockIdx.x, t = threadIdx.x & 63, lane = threadIdx.x >> 6;
   double acc = 0.0;
-  for (int k = 0; k < nchunk; ++k) acc += static_cast<double>(partial[(static_cast<long long>(b) * nchunk + k) * 64 + t]);
-  sums[static_cast<long long>(b) * 64 + t] = acc;
+  for (int c = lane; c < nchunk; c += kGnLanes)
+    acc += static_cast<double>(partial[(static_cast<long long>(b) * nchunk + c) * 64 + t]);
+  s_acc[lane][t] = acc;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    const int g = threadIdx.x;
+    double s = 0.0, q = 0.0;
+#pragma unroll
+    for (int l = 0; l < kGnLanes; ++l) s += s_acc[l][2 * g], q += s_acc[l][2 * g + 1];
+    // sum (x) = s + n k,  sum (x^2) = q + 2 k s + n k^2  (n = samples in the group)
+    const double k = x[static_cast<long long>(b) * P * C + g * (C / 32)];
+    const double n = static_cast<double>(P) * (C / 32);
+    sums[(static_cast<long long>(b) * 32 + g) * 2] = s + n * k;
+    sums[(static_cast<long long>(b) * 32 + g) * 2 + 1] = q + 2.0 * k * s + n * k * k;
+  }
 }
 
 // im2col with the producer fused in:  A[(b, y, x), (ky, kx, c)] = f(src[b, (y+ky-pad)/up, (x+kx-pad)/up, c])  (0 outside)
@@ -210,12 +236,13 @@ int mdt_vae_post_quant(const float* z, const float* W, const float* bias, float 
 }
 
 int mdt_vae_gn_stats(const float* x, double* sums, float* scratch, int B, int P, int C, void* stream) {
-  if (!x || !sums || !scratch || B <= 0 || P <= 0 || C % 128 || C > 512) return MDT_ERR_ARG;  // 4..16 channels / group
+  // 4, 8 or 16 channels per group: the partial kernel's 8 threads per group (C = 384 would leave slots unwritten)
+  if (!x || !sums || !scratch || B <= 0 || P <= 0 || (C != 128 && C != 256 && C != 512)) return MDT_ERR_ARG;
   if (reinterpret_cast<uintptr_t>(x) & 15) return MDT_ERR_ARG;
   const int nchunk = (P + kGnPix - 1) / kGnPix;
   dim3 block(C / 4, 256 / (C / 4)), grid(nchunk, B);
   vae_gn_partial_kernel<<<grid, block, 0, VS(stream)>>>(x, scratch, P, C);
-  vae_gn_finish_kernel<<<B, 64, 0, VS(stream)>>>(scratch, sums, nchunk);
+  vae_gn_finish_kernel<<<B, kGnLanes * 64, 0, VS(stream)>>>(x, scratch, sums, nchunk, P, C);
   return vae_status();
 }
 

@@ -1,6 +1,7 @@
 """Per-kernel parity (GPU): every C-ABI kernel against a plain PyTorch fp32 reference of the same op fed the SAME
 bf16-rounded inputs.  Tolerances are stated per test: fp32-accumulate kernels 1e-3 relative to the output scale,
-bf16-output kernels 1 bf16 ulp (2^-8) relative; the integer mask path is bit-exact."""
+bf16-output kernels 1 bf16 ulp (2^-8) relative; the integer mask path is bit-exact.  The SD-VAE kernels (`mdt_vae_*`)
+and the GEMM at the VAE's shapes are in test_vae_kernels_gpu.py."""
 import math
 import os
 
@@ -416,6 +417,20 @@ def test_heun_and_adamw(ops):
     close(w.cpu(), wr, 1e-6, "adamw w")
     close(ema.cpu(), er, 1e-6, "ema")
     close(v.cpu(), vr, 1e-4, "adamw v")
+    assert torch.equal(w16, w.to(torch.bfloat16))
+    # the bf16-gradient variant (mdt_adamw_ema_g16, after a bf16 all-reduce) on a grid capped at 3 blocks: 3 x 256
+    # threads x 4 elements per pass, so the grid-stride loop wraps 4 times over n = 10000
+    w = torch.randn(n, device=dev())
+    g16 = (torch.randn(n, device=dev()) * 0.01).to(torch.bfloat16)
+    m, v = torch.zeros(n, device=dev()), torch.zeros(n, device=dev())
+    ema = w.clone()
+    wr, mr, vr, er = w.cpu().clone(), m.cpu().clone(), v.cpu().clone(), ema.cpu().clone()
+    for step in (1, 2, 3):
+        ops.adamw_ema(w, g16, m, v, ema, w16, n, 1e-4, step, grad_scale=0.5, max_blocks=3)
+        O.adamw_ema_step(wr, g16.float().cpu() * 0.5, mr, vr, er, step)
+    close(w.cpu(), wr, 1e-6, "adamw g16 w")
+    close(ema.cpu(), er, 1e-6, "g16 ema")
+    close(v.cpu(), vr, 1e-4, "adamw g16 v")
     assert torch.equal(w16, w.to(torch.bfloat16))
 
 
